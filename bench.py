@@ -4,7 +4,7 @@
 N=16384, 5x60-bit primes, 61 ciphertext ops) on N B200s, plus the NTT HBM GB/s
 roofline line.  See the driver contract in the task description.
 
-  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+  python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 * our arm: the product path only (eva_b200 -> C-ABI -> CUDA); inputs/keys are
   synthetic uniform residues (every kernel is data-independent integer work).
@@ -26,6 +26,7 @@ ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
 WORKLOAD = "sobel"          # workloads/sobel.json: the reference compiler's output for examples/image_processing.py
 METRIC = "ciphertext-ops/sec"
+DUMP_BYTES = 60 * 10 ** 6   # --dump-outputs: all files together (npy headers aside) stay below 64 MB
 
 
 def load_workload(name):
@@ -126,7 +127,24 @@ def multi_seed(rank, index):
     return multi.instance_seed(rank, index)
 
 
-def measure_workload(args, wl, steps, rank, world, local):
+def dump_outputs(outdir, wl, d, outs, budget):
+    """The output ciphertexts that the last timed step handed to the caller (execute_batch_result: one valuation per
+    instance), as DIR/<workload>_<output>.npy, float64 [instances][polys][ell][coefficients][2]: every residue (< 2^60)
+    split exactly into its high and low 30 bits.  Above `budget` bytes per workload, a fixed seeded choice of
+    coefficient indices (the same in every run) is kept."""
+    os.makedirs(outdir, exist_ok=True)
+    names = sorted(d["outputs"])
+    for name in names:
+        arr = np.stack([np.asarray(o.get(name)[1]) for o in outs]).astype(np.uint64)
+        per_coeff = arr.size // arr.shape[-1] * 16
+        keep = max(1, min(arr.shape[-1], budget // len(names) // per_coeff))
+        if keep < arr.shape[-1]:
+            arr = arr[..., np.sort(np.random.default_rng(0).choice(arr.shape[-1], keep, replace=False))]
+        split = np.stack([arr >> np.uint64(30), arr & np.uint64((1 << 30) - 1)], axis=-1).astype(np.float64)
+        np.save(os.path.join(outdir, "%s_%s.npy" % (wl, name)), split)
+
+
+def measure_workload(args, wl, steps, rank, world, local, dump_budget=0):
     """device-resident value, e2e through execute_batch and single-instance latency of one workload"""
     import torch
     import torch.distributed as dist
@@ -251,6 +269,8 @@ def measure_workload(args, wl, steps, rank, world, local):
     t_e2e = time.perf_counter() - t0
     barrier()
     clocks = sampler.finish()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, wl, d, outs, dump_budget)
     h2d = sum(ct.nbytes for ct, _ in cts.values()) * B
     okind, oarr, _ = outs[0].get(list(d["outputs"].keys())[0])
     d2h = int(oarr.nbytes) * B
@@ -298,15 +318,16 @@ def run_ours(args):
     torch.cuda.set_device(local)
     if world > 1:
         dist.init_process_group("nccl", device_id=torch.device("cuda", local))
-    result, pub, main = measure_workload(args, args.workload, args.steps, rank, world, local)
-    if world == 1 and not args.no_extras:
-        # BASELINE configs 1 and 4 next to the headline (config 3): same measurement, fewer steps
+    extra_workloads = [] if (world > 1 or args.no_extras) else [n for n in ("harris", "polynomial") if n != args.workload]
+    dump_budget = DUMP_BYTES // (1 + len(extra_workloads))
+    result, pub, main = measure_workload(args, args.workload, args.steps, rank, world, local, dump_budget)
+    if extra_workloads:
+        # BASELINE configs 1 and 4 next to the headline (config 3): the same measurement
         extras = {}
-        for name in ("harris", "polynomial"):
-            if name != args.workload:
-                r, _, _ = measure_workload(args, name, max(5, args.steps // 5), rank, world, local)
-                extras[name] = {"workload": r["config"]["workload"], "value": r["value"], "unit": "ops/s", "ms_per_step": r["ms_per_step"],
-                                "e2e_value": r["e2e"]["value"], "single_instance": r["single_instance"]}
+        for name in extra_workloads:
+            r, _, _ = measure_workload(args, name, args.steps, rank, world, local, dump_budget)
+            extras[name] = {"workload": r["config"]["workload"], "value": r["value"], "unit": "ops/s", "ms_per_step": r["ms_per_step"],
+                            "e2e_value": r["e2e"]["value"], "single_instance": r["single_instance"]}
         result["other_workloads"] = extras
     if world > 1 and not args.no_dag_sharded:
         # north_star's other multi-GPU mode: ONE compiled program sharded over the GPUs (BASELINE configs 4 and 5)
@@ -314,7 +335,7 @@ def run_ours(args):
         import dagshard_bench
         shard_res = []
         for wl in ("wide4096", "harris"):
-            shard_res.append(dagshard_bench.measure(wl, rank, world, local, steps=20, warmup=3, quiet=True))
+            shard_res.append(dagshard_bench.measure(wl, rank, world, local, steps=args.steps, warmup=3, quiet=True))
         result["dag_sharded"] = [{k: r.get(k) for k in ("workload", "cipher_ops", "ms_single_gpu", "ms_sharded", "speedup", "bit_identical", "auto_choice", "stages", "note") if k in r} for r in shard_res]
     if rank == 0:
         result["roofline"] = ntt_roofline(pub, b200.create_coeff_modulus(16384, [60] * 4), 16384, main.cuda_stream)   # always the BASELINE shape
@@ -449,9 +470,15 @@ def main():
     ap.add_argument("--no-extras", action="store_true", help="skip the Harris / polynomial lines (other_workloads)")
     ap.add_argument("--no-dag-sharded", action="store_true", help="N > 1: skip the DAG-sharded wide4096 / Harris measurement (dag_sharded)")
     ap.add_argument("--workload", default=WORKLOAD, help="program under workloads/ (default: the BASELINE workload, sobel); e.g. harris")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="after the timed steps, write the outputs of the last e2e step of every workload as DIR/<workload>_<output>.npy "
+                         "(rank 0, replica workloads; not the N > 1 dag_sharded runs; nothing with --impl reference, whose CPU arm "
+                         "runs other inputs)")
     ap.add_argument("--ntt-cluster", type=int, default=None, help="CTAs per residue transform (1, 2, 4); default: library default")
     args = ap.parse_args()
     if args.impl == "reference":
+        if args.dump_outputs:
+            print("bench.py: --dump-outputs writes nothing with --impl reference", file=sys.stderr)
         run_reference(args)
     else:
         run_ours(args)

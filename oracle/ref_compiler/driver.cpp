@@ -55,6 +55,7 @@ int main() {
   std::map<long, Term::Ptr> T;
   std::unordered_map<std::string, std::string> cfg;
   std::map<std::string, std::vector<double>> evalInputs;
+  bool evaluate = false;   // print reference_outputs (also for a program without inputs)
   std::string line;
   uint32_t scale = 0, range = 0;
   while (std::getline(std::cin, line)) {
@@ -75,6 +76,7 @@ int main() {
     else if (cmd == "scales") is >> scale;
     else if (cmd == "ranges") is >> range;
     else if (cmd == "config") { std::string k, v; is >> k >> v; cfg[k] = v; }
+    else if (cmd == "evaluate") evaluate = true;
     else if (cmd == "evalinput") { std::string name; size_t n; is >> name >> n; std::vector<double> v(n); for (auto &x : v) is >> x; evalInputs[name] = v; }
   }
   // what python/eva/wrapper.cpp:48-68 set_output_ranges / set_input_scales do
@@ -105,7 +107,7 @@ int main() {
     Dumper d(cp);
     ProgramTraversal(cp).forwardPass(d);
     std::cout << d.out.str() << "\n]";
-    if (!evalInputs.empty()) {  // reference (plaintext) semantics: eva/eva.cpp:11-21
+    if (evaluate || !evalInputs.empty()) {  // reference (plaintext) semantics: eva/eva.cpp:11-21
       Valuation in;
       for (auto &e : evalInputs) in[e.first] = e.second;
       ReferenceExecutor ex(cp);
